@@ -170,8 +170,25 @@ def test_lm_wcpe_c1_matches_oracle():
     # (tools/wcpe_trace.py).  Compared while the damped system is well posed: the first five iterations.
     st = s.optimize(max_iterations=5); so = o.optimize(max_iterations=5)
     assert st["iterations"] == so["iterations"] == 5 and st["inner_iterations"] == so["inner_iterations"]
-    assert abs(st["error_final"] - so["error_final"]) <= 1e-3*so["error_final"]
     assert st["error_final"] < 2e-3*st["error_initial"]
+    # Both sides accumulate the reduced system with atomics, so each run differs from the next in the last bits, and along
+    # the gauge direction a step amplifies that by ~1/lambda: after five chained steps two runs of the SAME implementation
+    # differ by up to ~1e-3 in chi^2, so a comparison of the two trajectories' ends fails at random.  The five iterations
+    # are compared one at a time instead, the oracle taking each step from the GPU's iterate at the GPU's lambda.  Measured
+    # on a B200, GPU against oracle from equal inputs: <= 1.1e-5 relative while lambda >= 1e-8 (steps 1-4), <= 2.5e-4 for
+    # the fifth step (lambda 1e-9); the oracle against itself on 1 and 8 threads: <= 6e-6.
+    from dynosam_b200.binding import default_params
+    s = _solver(p); o = _oracle(p)
+    lam = default_params().lambda_initial
+    for it in range(5):
+        pose, point, _ = s.values()
+        o.pose[:] = pose; o.point[:] = point
+        st = s.optimize(max_iterations=1, lambda_initial=lam); so = o.optimize(max_iterations=1, lambda_initial=lam)
+        assert st["iterations"] == so["iterations"] == 1 and st["inner_iterations"] == so["inner_iterations"], it
+        assert abs(st["error_initial"] - so["error_initial"]) <= REL_CHI2*so["error_initial"], it
+        tol = 1e-4 if lam > 5e-9 else 1e-3          # lambda 1e-5 ... 1e-8, then 1e-9
+        assert abs(st["error_final"] - so["error_final"]) <= tol*so["error_final"], (it, st["error_final"], so["error_final"])
+        lam = st["lambda_final"]
 
 
 def test_damped_solve_every_factor_type():

@@ -1,4 +1,4 @@
-import sys; sys.path.insert(0,'/root/repo')
+import os, sys; sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
 from dynosam_b200 import synth
 from dynosam_b200.binding import Solver
