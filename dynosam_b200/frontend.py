@@ -13,7 +13,8 @@ LIB_PATH = os.path.join(_HERE, "libdynofront.so")
 EXPORTS = ["dynofront_create", "dynofront_destroy", "dynofront_last_error", "dynofront_set_frame", "dynofront_track_dynamic",
            "dynofront_sample_candidates", "dynofront_propagate_mask", "dynofront_klt_track", "dynofront_klt_track_fb",
            "dynofront_klt_last_min_eig", "dynofront_stereo_track", "dynofront_track_static_flow", "dynofront_next_frame", "dynofront_pin_host", "dynofront_unpin_host",
-           "dynofront_get_motion_mask", "dynofront_get_pyramid_level"]
+           "dynofront_get_motion_mask", "dynofront_get_pyramid_level", "dynofront_sample_dynamic", "dynofront_anms_range_tree",
+           "dynofront_anms_tie_order"]
 
 
 class TrackParamsC(C.Structure):
@@ -68,6 +69,11 @@ def load():
         L.dynofront_pin_host.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t]
         L.dynofront_unpin_host.argtypes = [C.c_void_p, C.c_void_p]
         L.dynofront_get_motion_mask.argtypes = [C.c_void_p, C.c_void_p]
+        L.dynofront_sample_dynamic.argtypes = [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_int32, C.c_float, C.POINTER(TrackParamsC),
+                                               C.POINTER(C.c_int64)] + [C.c_void_p]*8 + [C.c_int64, C.POINTER(C.c_float)]
+        L.dynofront_anms_range_tree.argtypes = [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_float, C.c_int32, C.c_int32,
+                                                C.c_void_p, C.c_void_p]
+        L.dynofront_anms_tie_order.argtypes = [C.c_int32, C.c_void_p]
         L.dynofront_get_pyramid_level.argtypes = [C.c_void_p, C.c_int32, C.c_int32, C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.c_void_p, C.c_void_p]
         _LIB = L
     return _LIB
@@ -79,6 +85,14 @@ def _p(a):
 
 class FrontendError(RuntimeError):
     pass
+
+
+def anms_tie_order(n):
+    """Walk order of n equal responses (cv::sortIdx(zeros(1, n), SORT_EVERY_ROW | SORT_DESCENDING)); host only."""
+    out = np.zeros(int(n), np.int32)
+    if load().dynofront_anms_tie_order(int(n), _p(out)) != 0:
+        raise FrontendError(f"dynofront_anms_tie_order({n}) failed")
+    return out
 
 
 class FeatureTrackerGPU:
@@ -154,6 +168,42 @@ class FeatureTrackerGPU:
         pc = prm.c()
         self._ck(self.lib.dynofront_sample_candidates(self.h, n, _p(objs), C.byref(pc), _p(counts), _p(offs), _p(zero), _p(idx), cap))
         return {int(o): idx[offs[i]:offs[i] + counts[i]].copy() for i, o in enumerate(objs)}, {int(o): int(zero[i]) for i, o in enumerate(objs)}
+
+    def sample_dynamic(self, objects, num_track, prm: TrackParams, next_tracklet_id: int, max_features=200, tolerance=0.01, capacity=None):
+        """FeatureTracker::sampleDynamic in one call: candidate scan, RangeTree ANMS with K = max(max_features - num_track, 0)
+        per object, new features.  Returns a dict: per object (order of `objects`) candidates / zero_flow / selected /
+        offset, per feature keypoint / flow / predicted (n, 2) float64, tracklet int64, object int32, and next_tracklet_id."""
+        objs = np.ascontiguousarray(objects, dtype=np.int32); n = objs.shape[0]
+        nt = np.ascontiguousarray(num_track, dtype=np.int32)
+        assert nt.shape == (n,)
+        cap = int(capacity if capacity is not None else max(int(max_features), 0)*n + 64)
+        cand = np.zeros(n, np.int32); zero = np.zeros(n, np.int32); sel = np.zeros(n, np.int32); off = np.zeros(n, np.int32)
+        kp = np.zeros((cap, 2)); fl = np.zeros((cap, 2)); pk = np.zeros((cap, 2)); tid = np.zeros(cap, np.int64)
+        nid = C.c_int64(int(next_tracklet_id)); pc = prm.c(); ms = C.c_float()
+        st = self.lib.dynofront_sample_dynamic(self.h, n, _p(objs), _p(nt), int(max_features), float(tolerance), C.byref(pc), C.byref(nid),
+                                               _p(cand), _p(zero), _p(sel), _p(off), _p(kp), _p(fl), _p(pk), _p(tid), cap, C.byref(ms))
+        if st == -1 and int(sel.sum()) > cap and capacity is None:          # more features than the default room: once more, large enough
+            return self.sample_dynamic(objects, num_track, prm, next_tracklet_id, max_features, tolerance, capacity=int(sel.sum()))
+        self._ck(st)
+        self.last_ms = ms.value
+        m = int(sel.sum())
+        return dict(candidates=cand, zero_flow=zero, selected=sel, offset=off, keypoint=kp[:m], flow=fl[:m], predicted=pk[:m], tracklet=tid[:m],
+                    object=np.repeat(objs, sel), next_tracklet_id=nid.value)
+
+    def anms_range_tree(self, lists, num_ret_points, tolerance=0.01, cols=None, rows=None):
+        """AdaptiveNonMaximumSuppression(RangeTree) on several lists of float (x, y) in one launch (the trackDynamicKLT call
+        site).  lists: sequence of (n_l, 2) arrays in the caller's order; num_ret_points: K per list.  Returns a list of
+        int32 arrays: the selected indices into each list, in selection order."""
+        arrs = [np.ascontiguousarray(a, dtype=np.float32).reshape(-1, 2) for a in lists]
+        counts = np.array([len(a) for a in arrs], np.int32)
+        xy = np.ascontiguousarray(np.concatenate(arrs) if arrs else np.zeros((0, 2), np.float32), dtype=np.float32)
+        K = np.ascontiguousarray(num_ret_points, dtype=np.int32).reshape(-1)
+        assert K.shape == counts.shape
+        idx = np.zeros(max(len(xy), 1), np.int32); nsel = np.zeros(len(arrs), np.int32)
+        self._ck(self.lib.dynofront_anms_range_tree(self.h, len(arrs), _p(counts), _p(xy), _p(K), float(tolerance), int(cols or self.W),
+                                                    int(rows or self.H), _p(idx), _p(nsel)))
+        offs = np.concatenate([[0], np.cumsum(counts)[:-1]]).astype(np.int64) if len(arrs) else []
+        return [idx[o:o + k].copy() for o, k in zip(offs, nsel)]
 
     def propagate_mask(self, prev_pred_kp, prev_label, prev_mask, prev_flow, current_mask, prm: TrackParams, min_votes=150):
         kp = np.ascontiguousarray(prev_pred_kp, dtype=np.float64).reshape(-1, 2)

@@ -17,6 +17,7 @@
 #include <vector>
 
 #include "../../include/dynofront.h"
+#include "anms.cuh"
 
 #define FCK(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { h->err = std::string(#call) + ": " + cudaGetErrorString(e_); return -3; } } while (0)
 
@@ -42,6 +43,11 @@ struct dynofront_ctx {
   int sf_cap = 0, sf_cells = 0; double* sf_kp = nullptr; int32_t* sf_age = nullptr; uint8_t* sf_use = nullptr; int32_t* sf_det = nullptr;
   int *sf_cell = nullptr, *sf_win = nullptr, *sf_win2 = nullptr, *sf_cnt = nullptr; uint8_t* sf_pass = nullptr; uint8_t* sf_acc = nullptr; double* sf_out = nullptr;
   int32_t* sf_oage = nullptr; long long* sf_otid = nullptr;
+  // sampleDynamic on the device (candidate lists, ANMS scratch, per-object plan) and batched ANMS of float lists
+  int *sd_idx = nullptr, *sd_off = nullptr, *sd_K = nullptr, *sd_sel = nullptr, *sd_out = nullptr, *sd_nsel = nullptr; float2* sd_pts = nullptr;
+  uint32_t* sd_bm = nullptr; long long* sd_bm_off = nullptr; unsigned char *sd_host = nullptr, *sd_host_dev = nullptr; long long sd_host_cap = -1;
+  int an_cap = 0, an_lists = 0; long long an_bm_cap = 0; float* an_xy = nullptr; float2* an_pts = nullptr; int *an_sel = nullptr, *an_out = nullptr;
+  int *an_meta = nullptr; uint32_t* an_bm = nullptr; long long* an_bm_off = nullptr; int anms_smem = 0;
   cudaEvent_t e0 = nullptr, e1 = nullptr;
   std::vector<void*> allocs;
 };
@@ -229,6 +235,38 @@ __global__ void __launch_bounds__(ST_TILE) sc_scatter_kernel(size_t npx, int W, 
     for (int w = 0; w < warp; w++) base += wc[w][s];
     const long long dst = (long long)obj_off[s] + tile_off[(size_t)blockIdx.x*ST_MAXOBJ + s] + base + myrank;
     if (dst < capacity) indices[dst] = (int)p;
+  }
+}
+
+// ---------------------------------------------------------------------------------------------------- sampleDynamic tail
+// FeatureTracker.cc:955-1015 after the scan: per object K = max(max_features - num_track, 0) (:966-969), the candidate
+// lists (ascending pixel index, the order of a serial run of the reference's fill) through suppressNonMax(RangeTree),
+// then the new features.  Tracklet ids follow the order of objects[] (the reference's parallel for_each over a hash map
+// leaves that order undefined), as dynofront_track_dynamic hands ids out in array order.
+__global__ void sd_plan_kernel(int nobj, const int* obj_tot, const int* num_track, int max_features, int* off, int* K) {
+  if (threadIdx.x != 0) return;
+  int run = 0;
+  for (int o = 0; o < nobj; o++) { off[o] = run; run += obj_tot[o]; K[o] = max(max_features - num_track[o], 0); }
+}
+// one CTA per object: exclusive scan of the selected counts over the objects gives the first feature / tracklet id;
+// age 0, key-point (j, i), measured flow float -> double, predicted key-point = key-point + flow.  Writes straight into
+// the mapped host staging buffer, so only the selected features cross PCIe.
+__global__ void sd_construct_kernel(int nobj, const int* off, const int* tot, const int* zero, const int* nsel, const int* sel, const int* idx, int W,
+                                    const float* __restrict__ flow, long long capacity, long long base_id, int32_t* stats, double* feat, long long* tid) {
+  const int o = blockIdx.x;
+  int pre = 0;
+  for (int q = 0; q < o; q++) pre += nsel[q];
+  const int ns = nsel[o];
+  if (threadIdx.x == 0) { stats[o] = tot[o]; stats[ST_MAXOBJ + o] = zero[o]; stats[2*ST_MAXOBJ + o] = ns; stats[3*ST_MAXOBJ + o] = pre; }
+  for (int t = threadIdx.x; t < ns; t += blockDim.x) {
+    const long long f = (long long)pre + t;
+    if (f >= capacity) break;
+    const int p = idx[off[o] + sel[off[o] + t]];
+    const int i = p / W, j = p % W;
+    const double fx = (double)flow[2*(size_t)p], fy = (double)flow[2*(size_t)p + 1];
+    double* r = feat + 6*f;
+    r[0] = (double)j; r[1] = (double)i; r[2] = fx; r[3] = fy; r[4] = (double)j + fx; r[5] = (double)i + fy;
+    tid[f] = base_id + f;
   }
 }
 
@@ -537,6 +575,7 @@ int dynofront_destroy(dynofront_handle h) {
   for (void* p : h->allocs) cudaFree(p);
   if (h->e0) cudaEventDestroy(h->e0); if (h->e1) cudaEventDestroy(h->e1);
   if (h->s) cudaStreamDestroy(h->s);
+  if (h->sd_host) cudaFreeHost(h->sd_host);
   delete h; return 0;
 }
 int dynofront_set_frame(dynofront_handle h, const float* flow, const int32_t* motion_mask, const uint8_t* detection_mask) {
@@ -942,6 +981,148 @@ int dynofront_track_static_flow(dynofront_handle h, int32_t n_prev, const double
   FCK(cudaGetLastError());
   *next_tracklet_id += cnt[1];
   if (n_tracked) *n_tracked = cnt[0]; if (n_detected) *n_detected = cnt[1];
+  return 0;
+}
+
+// ---------------------------------------------------------------------------------------------------- ANMS / sampleDynamic host side
+static int anms_prepare(dynofront_ctx* h) {       // the ANMS kernel may use all the shared memory a block can opt into
+  if (h->anms_smem) return 0;
+  int optin = 0; cudaFuncAttributes fa;
+  FCK(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, h->dev));
+  FCK(cudaFuncGetAttributes(&fa, anms_range_tree_kernel));
+  const int dyn = (optin - (int)fa.sharedSizeBytes) & ~15;
+  FCK(cudaFuncSetAttribute(anms_range_tree_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, dyn));
+  h->anms_smem = dyn;
+  return 0;
+}
+static int sd_scratch(dynofront_ctx* h, long long capacity) {
+  if (anms_prepare(h)) return -3;
+  const size_t npx = (size_t)h->W*h->H;
+  if (!h->sd_idx) {
+    const long long bmw = (long long)((h->W + 31)/32)*h->H;       // a bounding box of cells is at most the whole image
+    int rc = 0;
+    rc |= falloc(h, &h->sd_idx, npx); rc |= falloc(h, &h->sd_off, ST_MAXOBJ); rc |= falloc(h, &h->sd_K, ST_MAXOBJ); rc |= falloc(h, &h->sd_nsel, ST_MAXOBJ);
+    rc |= falloc(h, &h->sd_sel, 2*npx); rc |= falloc(h, &h->sd_out, npx); rc |= falloc(h, &h->sd_pts, npx);
+    rc |= falloc(h, &h->sd_bm, (size_t)(ST_MAXOBJ*bmw)); rc |= falloc(h, &h->sd_bm_off, ST_MAXOBJ);
+    if (rc) return -3;
+    std::vector<long long> bo(ST_MAXOBJ);
+    for (int o = 0; o < ST_MAXOBJ; o++) bo[o] = o*bmw;
+    FCK(cudaMemcpy(h->sd_bm_off, bo.data(), ST_MAXOBJ*sizeof(long long), cudaMemcpyHostToDevice));
+  }
+  if (capacity > h->sd_host_cap) {                 // mapped pinned staging: inputs, per-object stats, features
+    if (h->sd_host) { cudaFreeHost(h->sd_host); h->sd_host = h->sd_host_dev = nullptr; h->sd_host_cap = -1; }
+    const long long cap = std::max<long long>(capacity, 1024);
+    FCK(cudaHostAlloc((void**)&h->sd_host, 6*ST_MAXOBJ*4 + (size_t)cap*(6*8 + 8), cudaHostAllocMapped));
+    FCK(cudaHostGetDevicePointer((void**)&h->sd_host_dev, h->sd_host, 0));
+    h->sd_host_cap = cap;
+  }
+  return 0;
+}
+
+int dynofront_sample_dynamic(dynofront_handle h, int32_t nobj, const int32_t* objects, const int32_t* num_track, int32_t max_features,
+                             float tolerance, const dynofront_track_params* prm, int64_t* next_tracklet_id, int32_t* candidates,
+                             int32_t* zero_flow, int32_t* selected, int32_t* selected_offset, double* keypoint, double* flow_out,
+                             double* predicted_keypoint, int64_t* tracklet, int64_t capacity, float* ms_device) {
+  if (!h || !prm || !next_tracklet_id || nobj < 0 || nobj > ST_MAXOBJ || capacity < 0) return -1;
+  if (nobj && (!objects || !num_track || !candidates || !selected || !selected_offset)) { h->err = "null per-object array"; return -1; }
+  if (capacity && (!keypoint || !flow_out || !predicted_keypoint || !tracklet)) { h->err = "null per-feature array"; return -1; }
+  cudaSetDevice(h->dev);
+  if (sd_scratch(h, capacity)) return -3;
+  const size_t npx = (size_t)h->W*h->H; const int ntiles = (int)((npx + ST_TILE - 1)/ST_TILE);
+  int32_t* in = (int32_t*)h->sd_host; int32_t* stats = in + 2*ST_MAXOBJ;
+  int32_t* stats_dev = (int32_t*)h->sd_host_dev + 2*ST_MAXOBJ;
+  double* feat = (double*)(h->sd_host + 6*ST_MAXOBJ*4); long long* tid = (long long*)(feat + 6*h->sd_host_cap);
+  double* feat_dev = (double*)(h->sd_host_dev + 6*ST_MAXOBJ*4); long long* tid_dev = (long long*)(feat_dev + 6*h->sd_host_cap);
+  std::memcpy(in, objects, (size_t)nobj*4); std::memcpy(in + ST_MAXOBJ, num_track, (size_t)nobj*4);
+  FCK(cudaEventRecord(h->e0, h->s));
+  if (!h->det_work_valid) prepare_det_work(h);
+  if (nobj > 0) {
+    FCK(cudaMemcpyAsync(h->d_objs, in, (size_t)nobj*4, cudaMemcpyHostToDevice, h->s));
+    FCK(cudaMemcpyAsync(h->sd_K, in + ST_MAXOBJ, (size_t)nobj*4, cudaMemcpyHostToDevice, h->s));
+    FCK(cudaMemsetAsync(h->d_zero, 0, ST_MAXOBJ*4, h->s));
+    sc_count_kernel<<<ntiles, ST_TILE, 0, h->s>>>(npx, h->W, h->H, h->det_work, h->mask, h->flow, h->d_objs, nobj, *prm, h->tile_cnt, h->d_zero);
+    sc_scan_kernel<<<1, ST_MAXOBJ, 0, h->s>>>(ntiles, nobj, h->tile_cnt, h->obj_tot);
+    sd_plan_kernel<<<1, 32, 0, h->s>>>(nobj, h->obj_tot, h->sd_K, max_features, h->sd_off, h->sd_K);
+    sc_scatter_kernel<<<ntiles, ST_TILE, 0, h->s>>>(npx, h->W, h->H, h->det_work, h->mask, h->flow, h->d_objs, nobj, *prm, h->tile_cnt, h->sd_off,
+                                                    h->sd_idx, (long long)npx);
+    AnmsArgs a{h->sd_off, h->obj_tot, h->sd_K, nullptr, h->sd_idx, h->W, tolerance, h->W, h->H, h->sd_pts, h->sd_bm, h->sd_bm_off,
+               h->sd_sel, (long long)npx, h->sd_out, h->sd_nsel, h->anms_smem};
+    anms_range_tree_kernel<<<nobj, ANMS_THREADS, h->anms_smem, h->s>>>(a);
+    sd_construct_kernel<<<nobj, 128, 0, h->s>>>(nobj, h->sd_off, h->obj_tot, h->d_zero, h->sd_nsel, h->sd_out, h->sd_idx, h->W, h->flow,
+                                                capacity, (long long)*next_tracklet_id, stats_dev, feat_dev, tid_dev);
+  }
+  FCK(cudaEventRecord(h->e1, h->s));
+  FCK(cudaStreamSynchronize(h->s));
+  FCK(cudaGetLastError());
+  long long total = 0;
+  for (int o = 0; o < nobj; o++) {
+    candidates[o] = stats[o]; if (zero_flow) zero_flow[o] = stats[ST_MAXOBJ + o];
+    selected[o] = stats[2*ST_MAXOBJ + o]; selected_offset[o] = stats[3*ST_MAXOBJ + o]; total += selected[o];
+  }
+  if (ms_device) FCK(cudaEventElapsedTime(ms_device, h->e0, h->e1));
+  if (total > capacity) { h->err = "capacity < " + std::to_string(total) + " selected features"; return -1; }
+  for (long long f = 0; f < total; f++) {
+    keypoint[2*f] = feat[6*f]; keypoint[2*f + 1] = feat[6*f + 1]; flow_out[2*f] = feat[6*f + 2]; flow_out[2*f + 1] = feat[6*f + 3];
+    predicted_keypoint[2*f] = feat[6*f + 4]; predicted_keypoint[2*f + 1] = feat[6*f + 5]; tracklet[f] = tid[f];
+  }
+  *next_tracklet_id += total;
+  return 0;
+}
+
+int dynofront_anms_range_tree(dynofront_handle h, int32_t n_lists, const int32_t* counts, const float* xy, const int32_t* num_ret_points,
+                              float tolerance, int32_t cols, int32_t rows, int32_t* indices, int32_t* n_selected) {
+  if (!h || n_lists < 0 || (n_lists && (!counts || !num_ret_points || !n_selected))) return -1;
+  if (cols <= 0 || rows <= 0 || cols > 65535 || rows > 65535) { h->err = "cols / rows must be in [1, 65535] (u16 cells)"; return -1; }
+  cudaSetDevice(h->dev);
+  if (anms_prepare(h)) return -3;
+  std::vector<int> meta(4*(size_t)n_lists);         // off, count, K, (selected)
+  std::vector<long long> bm_off(std::max(n_lists, 1));
+  long long total = 0, bm_total = 0;
+  for (int l = 0; l < n_lists; l++) {
+    if (counts[l] < 0) { h->err = "negative list length"; return -1; }
+    meta[l] = (int)total; meta[n_lists + l] = counts[l]; meta[2*n_lists + l] = num_ret_points[l];
+    float bx0 = 65536.f, bx1 = -1.f, by0 = 65536.f, by1 = -1.f;
+    for (long long i = total; i < total + counts[l]; i++) {
+      const float x = xy[2*i], y = xy[2*i + 1];
+      if (!(x >= 0.f && x < 65536.f && y >= 0.f && y < 65536.f)) { h->err = "coordinates must lie in [0, 65536) (u16 cells)"; return -1; }
+      bx0 = std::min(bx0, x); bx1 = std::max(bx1, x); by0 = std::min(by0, y); by1 = std::max(by1, y);
+    }
+    total += counts[l];
+    if (total > INT32_MAX/2) { h->err = "too many points"; return -1; }
+    bm_off[l] = bm_total;                            // global bitmap only where the kernel cannot keep it in shared memory
+    if (counts[l] > 0) {
+      const long long words = (long long)((((int)bx1 - (int)bx0) >> 5) + 1)*((int)by1 - (int)by0 + 1);
+      if (4*words > h->anms_smem) bm_total += words;
+    }
+  }
+  if (n_lists == 0) return 0;
+  if (total > h->an_cap) {
+    const int cap = (int)std::max<long long>(2*total, 4096);
+    if (falloc(h, &h->an_xy, 2*(size_t)cap) || falloc(h, &h->an_pts, cap) || falloc(h, &h->an_sel, 2*(size_t)cap) || falloc(h, &h->an_out, cap)) return -3;
+    h->an_cap = cap;
+  }
+  if (n_lists > h->an_lists) {
+    const int cap = std::max(2*n_lists, 64);
+    if (falloc(h, &h->an_meta, 4*(size_t)cap) || falloc(h, &h->an_bm_off, cap)) return -3;
+    h->an_lists = cap;
+  }
+  if (bm_total > h->an_bm_cap) { if (falloc(h, &h->an_bm, (size_t)bm_total)) return -3; h->an_bm_cap = bm_total; }
+  FCK(cudaMemcpyAsync(h->an_meta, meta.data(), meta.size()*4, cudaMemcpyHostToDevice, h->s));
+  FCK(cudaMemcpyAsync(h->an_bm_off, bm_off.data(), (size_t)n_lists*8, cudaMemcpyHostToDevice, h->s));
+  if (total) FCK(cudaMemcpyAsync(h->an_xy, xy, 2*(size_t)total*4, cudaMemcpyHostToDevice, h->s));
+  AnmsArgs a{h->an_meta, h->an_meta + n_lists, h->an_meta + 2*n_lists, h->an_xy, nullptr, 0, tolerance, cols, rows, h->an_pts, h->an_bm, h->an_bm_off,
+             h->an_sel, (long long)h->an_cap, h->an_out, h->an_meta + 3*n_lists, h->anms_smem};
+  anms_range_tree_kernel<<<n_lists, ANMS_THREADS, h->anms_smem, h->s>>>(a);
+  if (total && indices) FCK(cudaMemcpyAsync(indices, h->an_out, (size_t)total*4, cudaMemcpyDeviceToHost, h->s));
+  FCK(cudaMemcpyAsync(n_selected, h->an_meta + 3*n_lists, (size_t)n_lists*4, cudaMemcpyDeviceToHost, h->s));
+  FCK(cudaStreamSynchronize(h->s));
+  FCK(cudaGetLastError());
+  return 0;
+}
+
+int dynofront_anms_tie_order(int32_t n, int32_t* out) {
+  if (n < 0 || (n && !out)) return -1;
+  for (int k = 0; k < n; k++) out[k] = anms_tie_source(n, k);
   return 0;
 }
 

@@ -5,6 +5,9 @@
  * Replaces, with the same inputs / outputs and the same ordering semantics:
  *   dynofront_track_dynamic     FeatureTracker::trackDynamic        dynosam/src/frontend/vision/FeatureTracker.cc:339-498
  *   dynofront_sample_candidates FeatureTracker::sampleDynamic scan  FeatureTracker.cc:864-953
+ *   dynofront_sample_dynamic    FeatureTracker::sampleDynamic: scan, ANMS (RangeTree), new features  FeatureTracker.cc:864-1015
+ *   dynofront_anms_range_tree   AdaptiveNonMaximumSuppression(RangeTree)::suppressNonMax on equal responses
+ *                               (NonMaximumSupression.cc:45-93, anms.cc:278-362), as trackDynamicKLT calls it (:818-834)
  *   dynofront_propagate_mask    FeatureTracker::propogateMask       FeatureTracker.cc:1212-1359
  *   dynofront_track_static_flow ExternalFlowFeatureTracker::trackStatic / constructStaticFeature  StaticFeatureTracker.cc:70-220
  *   dynofront_klt_track_fb      KltFeatureTracker::trackPoints: forward + backward LK, round-trip test, label / border / age checks (:486-592)
@@ -65,6 +68,35 @@ int dynofront_track_dynamic(dynofront_handle h, int32_t n, const double* prev_pr
  * object skipped because a flow component is exactly 0.  capacity = size of indices. */
 int dynofront_sample_candidates(dynofront_handle h, int32_t n_objects, const int32_t* objects, const dynofront_track_params* prm,
                                 int32_t* counts, int32_t* offsets, int32_t* zero_flow, int32_t* indices, int64_t capacity);
+
+/* sampleDynamic as ONE call: the candidate scan above, then per object AdaptiveNonMaximumSuppression(RangeTree) with
+ * K = max(max_features - num_track[o], 0) and the given tolerance (0.01 in the reference) over the candidate list in
+ * ascending pixel order, then the new features (FeatureTracker.cc:955-1015).  Uses the detection mask left on the device
+ * by dynofront_track_dynamic (or the uploaded one); synchronises once, and only the selected features cross PCIe.
+ * Per object: candidates[o] (the scan's count), zero_flow[o] (may be NULL), selected[o] and selected_offset[o] (first
+ * row of the object's features; objects follow each other in the order of objects[]).  Per feature, in selection order:
+ * keypoint[f][2] = (col, row), flow[f][2] (float -> double), predicted_keypoint[f][2] = keypoint + flow and tracklet[f],
+ * counting up from *next_tracklet_id, which is updated.  New features have age 0.  K = 0 gives no features (the
+ * reference's K = 0 is undefined behaviour, DESIGN.md section 8f-4).  If more than `capacity` features are selected the
+ * call returns -1 with the per-object outputs filled in and *next_tracklet_id unchanged.  ms_device (may be NULL) = device
+ * time from the first to the last operation of the call. */
+int dynofront_sample_dynamic(dynofront_handle h, int32_t n_objects, const int32_t* objects, const int32_t* num_track, int32_t max_features,
+                             float tolerance, const dynofront_track_params* prm, int64_t* next_tracklet_id, int32_t* candidates,
+                             int32_t* zero_flow, int32_t* selected, int32_t* selected_offset, double* keypoint, double* flow,
+                             double* predicted_keypoint, int64_t* tracklet, int64_t capacity, float* ms_device);
+
+/* AdaptiveNonMaximumSuppression(RangeTree) on n_lists lists in one launch.  List l holds counts[l] points, stored one
+ * list after the other in xy[][2] (float, in the caller's order; all responses equal, so the walk order is cv::sortIdx's
+ * tie order, dynofront_anms_tie_order).  Coordinates must lie in [0, 65536) and cols / rows in [1, 65535]: the reference
+ * keeps u16 cells.  num_ret_points[l] = K (<= 0: nothing selected).  Writes n_selected[l] and, at the list's own offset in
+ * indices[], the selected points' indices within the list in selection order.  Bit-exact with the reference, including
+ * its binary search ending on the previous width's selection (which need not hold K points) and K = 1 selecting nothing.
+ * (Search boxes are not wrapped at 65536, where the reference's u16 bounds would.) */
+int dynofront_anms_range_tree(dynofront_handle h, int32_t n_lists, const int32_t* counts, const float* xy, const int32_t* num_ret_points,
+                              float tolerance, int32_t cols, int32_t rows, int32_t* indices, int32_t* n_selected);
+/* parity hook, host only (no device needed): the walk order of n equal responses, out[k] = input index of the k-th point
+ * = cv::sortIdx(zeros(1, n), SORT_EVERY_ROW | SORT_DESCENDING) */
+int dynofront_anms_tie_order(int32_t n, int32_t* out);
 
 /* propogateMask: previous-frame features (predicted key-point, label), previous mask / flow, current mask (in/out).
  * All three images NULL: streaming mode, the resident previous frame votes into the resident current motion mask in place. */
